@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Contract benchmark: audio samples/sec (fwd+bwd) of the dasp hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                    # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # the reference's own CPU path
     python bench.py --impl reference-cuda                                  # the reference's own PyTorch-CUDA path (1 GPU)
 
@@ -355,14 +355,17 @@ class Step:
         self.d = self.host[2].to(dev).requires_grad_(True)
         self.graph = None
         self.loss = None
+        self.y = None
         self.pool = pool
 
     def eager(self):
         for t in (self.x, self.p, self.d):
             t.grad = None
+        self.y = None
         y = chain(self.D, self.x, self.p, self.d)
         loss = y.pow(2).mean()
         loss.backward()
+        self.y = y.detach()
         return loss
 
     def capture(self, warm=3):
@@ -376,6 +379,7 @@ class Step:
         torch.cuda.synchronize(self.dev)
         for t in (self.x, self.p, self.d):
             t.grad = None
+        self.y = None
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, pool=self.pool):
             self.loss = self.eager()
@@ -383,6 +387,24 @@ class Step:
 
     def replay(self):
         self.graph.replay()
+
+
+DUMP_ITEMS = 32
+
+
+def dump_outputs(step, out_dir):
+    """Write what the last run of `step` computed as out_dir/<name>.npy (float32): the loss, dL/dp (bs, 49) and
+    dL/d(drive) (bs*2,) whole, and y and dL/dx (DUMP_ITEMS, 2, N) for the items picked by a fixed seeded
+    permutation of the batch (24.6 MB at N = 48000).  The inputs and the device noise are seeded, so the same
+    arguments give the same arrays from one run to the next."""
+    import numpy as np
+    torch = step.torch
+    items = torch.randperm(step.bs, generator=torch.Generator().manual_seed(0))[:DUMP_ITEMS].sort().values.to(step.dev)
+    arrays = {"loss": step.loss, "y": step.y[items], "x_grad": step.x.grad[items], "p_grad": step.p.grad,
+              "drive_grad": step.d.grad}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def own_launches_per_step(bs, chunk_items):
@@ -470,7 +492,13 @@ def main():
                                                                    "under weak scaling (BASELINE config: 1024)")
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"])
     ap.add_argument("--no-extras", action="store_true", help="skip sub-configs / reference_gpu / cpu_baseline / edges")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the outputs of the last one "
+                                                          "as DIR/<name>.npy (rank 0's shard when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200 only")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -498,6 +526,7 @@ def main():
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback exists)"
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
+    torch.cuda.manual_seed(1000 + rank)     # torch seeds its CUDA generator at random; the reverb draws its noise from it
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
@@ -563,6 +592,8 @@ def main():
     clocks = sampler.stop(wall0, wall1)
     value = samples_per_step * args.steps / (ms_max * 1e-3)
     loss_val = float(step.loss.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step, args.dump_outputs)        # before the end-to-end replays below overwrite the outputs
 
     # ---- end-to-end: pinned host inputs -> H2D -> graph replay -> D2H of loss and parameter gradients ----
     # Every step uploads ITS inputs from pinned host memory into a staging set on a copy stream (overlapping the

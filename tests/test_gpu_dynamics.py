@@ -43,16 +43,17 @@ def test_compressor_golden(cuda_device):
     import dasp_pytorch_b200 as D
     g = load_golden("compressor.npz")
     names = [str(s) for s in g["names"]]
+    s = int(g["t_stride"])         # per-sample reference arrays are stored at every s-th time index
     params = denorm(g["p01"], COMP_RANGES)
     y, dx, dp = run_with_grads(lambda xx, p: D.compressor(xx, SR, *p), g["x"], params, torch.float32, cuda_device)
     # item 0 has a 90 ms attack at N=4096: the reference time-aliases there (tests/test_oracle_golden.py)
-    assert peak_err(y, g["comp_y64"])[1:].max() < TOL
-    assert peak_err(dx, g["comp_dx64"])[1:].max() < TOL
+    assert peak_err(y[..., ::s], g["comp_y64"])[1:].max() < TOL
+    assert peak_err(dx[..., ::s], g["comp_dx64"])[1:].max() < TOL
     ref = [None if n == "release_ms" else torch.as_tensor(g[f"comp_d_{n}"]) for n in names]
     assert param_grad_err(dp, ref)[1:].max() < TOL
     y7 = D.compressor(torch.as_tensor(g["x"]).to(cuda_device), SR, *[p.to(cuda_device) for p in params],
                       lookahead_samples=7).cpu()
-    assert peak_err(y7, g["comp_la7_y64"])[1:].max() < TOL
+    assert peak_err(y7[..., ::s], g["comp_la7_y64"])[1:].max() < TOL
 
 
 @pytest.mark.parametrize("bs,chs,n", [(8, 2, 48000), (3, 1, 48000), (2, 3, 20000)])

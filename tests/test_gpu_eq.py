@@ -45,11 +45,12 @@ def test_eq_golden(cuda_device):
     import dasp_pytorch_b200 as D
     g = load_golden("parametric_eq.npz")
     names = [str(s) for s in g["names"]]
+    s = int(g["t_stride"])         # per-sample reference arrays are stored at every s-th time index
     params = denorm(g["p01"], eq_ranges())
     y, dx, dp = run_with_grads(lambda xx, p: D.parametric_eq(xx, SR, *p), g["x"], params, torch.float32, cuda_device)
     # item 0 (20 Hz low shelf at N=4096) is where the reference itself time-aliases; see test_oracle_golden
-    assert peak_err(y, g["eq_y64"])[1:].max() < TOL
-    assert peak_err(dx, g["eq_dx64"])[1:].max() < TOL
+    assert peak_err(y[..., ::s], g["eq_y64"])[1:].max() < TOL
+    assert peak_err(dx[..., ::s], g["eq_dx64"])[1:].max() < TOL
     ref = [torch.as_tensor(g[f"eq_d_{n}"]) for n in names]
     assert param_grad_err(dp, ref)[1:].max() < TOL
 

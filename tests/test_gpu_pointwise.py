@@ -13,26 +13,28 @@ pytestmark = pytest.mark.gpu
 def test_distortion_golden(cuda_device):
     import dasp_pytorch_b200 as D
     g = load_golden("pointwise.npz")
+    s = int(g["t_stride"])         # per-sample reference arrays are stored at every s-th time index
     y, dx, dp = run_with_grads(lambda x, p: D.distortion(x, 16000, p[0]), g["dist_x"], [g["dist_db"]],
                                torch.float32, cuda_device)
-    assert peak_err(y, g["dist_y64"]).max() < 1e-5        # tolerance: 1e-4 rel fp32 (north star); observed ~1e-7
-    assert peak_err(y, g["dist_y32"]).max() < 1e-5
-    assert peak_err(dx, g["dist_dx64"]).max() < 1e-5
+    assert peak_err(y[..., ::s], g["dist_y64"]).max() < 1e-5        # tolerance: 1e-4 rel fp32 (north star); observed ~1e-7
+    assert peak_err(y[..., ::s], g["dist_y32"]).max() < 1e-5
+    assert peak_err(dx[..., ::s], g["dist_dx64"]).max() < 1e-5
     assert np.allclose(dp[0].numpy(), g["dist_d_drive_db"], rtol=1e-4, atol=1e-9)
     # stereo: one drive per (item, channel) row
     y, dx, dp = run_with_grads(lambda x, p: D.distortion(x, SR, p[0]), g["dist2_x"], [g["dist2_db"]],
                                torch.float32, cuda_device)
-    assert peak_err(y, g["dist2_y64"]).max() < 1e-5
+    assert peak_err(y[..., ::s], g["dist2_y64"]).max() < 1e-5
     assert np.allclose(dp[0].numpy(), g["dist2_d_drive_db"], rtol=1e-4, atol=1e-9)
 
 
 def test_gain_golden(cuda_device):
     import dasp_pytorch_b200 as D
     g = load_golden("pointwise.npz")
+    s = int(g["t_stride"])
     y, dx, dp = run_with_grads(lambda x, p: D.gain(x, SR, p[0]), g["gain_x"], [g["gain_db"]], torch.float32,
                                cuda_device)
-    assert peak_err(y, g["gain_y64"]).max() < 1e-5
-    assert peak_err(dx, g["gain_dx64"]).max() < 1e-5
+    assert peak_err(y[..., ::s], g["gain_y64"]).max() < 1e-5
+    assert peak_err(dx[..., ::s], g["gain_dx64"]).max() < 1e-5
     assert np.allclose(dp[0].numpy(), g["gain_d_gain_db"], rtol=1e-4, atol=1e-9)
 
 
