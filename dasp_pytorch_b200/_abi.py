@@ -12,7 +12,7 @@ from ctypes import c_char_p, c_double, c_float, c_int, c_int64, c_uint64, c_void
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("DASP_LIB_PATH") or os.path.join(_HERE, "libdasp_b200.so")   # override: experiments only
+LIB_PATH = os.path.join(_HERE, "libdasp_b200.so")
 
 ABI_VERSION = 2
 
@@ -41,8 +41,6 @@ _SIGNATURES = {
     "dasp_compiled_arch": (c_int, []),
     "dasp_shutdown": (None, []),
     "dasp_debug_force_warps": (None, [c_int]),
-    "dasp_debug_eq_bwd_stages": (None, [c_int]),
-    "dasp_debug_reverb_path": (None, [c_int]),
     "dasp_debug_reverb_last_path": (c_int, []),
     "dasp_debug_reverb_flat_filterbank": (None, [c_int]),
     "dasp_denormalize": (c_int, [P, P, P, P, P, I64, I64, P]),

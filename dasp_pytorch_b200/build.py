@@ -15,8 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
-# experiments: DASP_NVCC_DEFS="-DDASP_EQ_E=7" DASP_LIB_SUFFIX=_e7 python -m dasp_pytorch_b200.build --force
-LIB = os.path.join(HERE, f"libdasp_b200{os.environ.get('DASP_LIB_SUFFIX', '')}.so")
+LIB = os.path.join(HERE, "libdasp_b200.so")
 SOURCES = ["abi.cu", "pointwise.cu", "stereo.cu", "dynamics.cu", "biquad.cu", "reverb.cu"]
 
 NVCC_FLAGS = [
@@ -24,6 +23,8 @@ NVCC_FLAGS = [
     "-O3", "-std=c++17", "-lineinfo",
     "-Xcompiler", "-fPIC,-O3,-Wall",
     "-Xptxas", "-v",
+    # compress every cubin in the fatbinary: the default heuristic leaves some large ones (reverb.cu: 9 MB) uncompressed
+    "-Xfatbin=-compress-all",
 ]
 
 
@@ -53,8 +54,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
     procs = []
     os.makedirs(os.path.join(HERE, "build"), exist_ok=True)
     for src in srcs:
-        obj = os.path.join(HERE, "build", os.path.basename(src) + os.environ.get("DASP_LIB_SUFFIX", "") + ".o")
-        cmd = [nvcc, *NVCC_FLAGS, *os.environ.get("DASP_NVCC_DEFS", "").split(), "-I", INCLUDE, "-I", CSRC, "-c", src, "-o", obj]
+        obj = os.path.join(HERE, "build", os.path.basename(src) + ".o")
+        cmd = [nvcc, *NVCC_FLAGS, "-I", INCLUDE, "-I", CSRC, "-c", src, "-o", obj]
         procs.append((src, cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
         objs.append(obj)
     for src, cmd, p in procs:

@@ -32,11 +32,6 @@ int sm_count() {
 
 static int g_forced_warps = 0;
 int debug_forced_warps() { return g_forced_warps; }
-static int g_reverb_path = 0;
-int debug_reverb_path() { return g_reverb_path; }
-
-static int g_eq_bwd_stages = 0;
-int debug_eq_bwd_stages() { return g_eq_bwd_stages; }
 static int g_flat_fb = 0;
 int debug_flat_filterbank() { return g_flat_fb; }
 
@@ -65,7 +60,7 @@ int dasp_abi_version(void) { return DASP_ABI_VERSION; }
 const char* dasp_last_error(void) { return dasp::g_err; }
 int dasp_compiled_arch(void) { return 1000; }
 void dasp_shutdown(void) { dasp::reverb_shutdown(); }
-void dasp_debug_force_warps(int warps) { dasp::g_forced_warps = (warps == 1 || warps == 2 || warps == 3 || warps == 4 || warps == 8 || warps == 16) ? warps : 0; }
+void dasp_debug_force_warps(int warps) { dasp::g_forced_warps = (warps == 1 || warps == 2 || warps == 4 || warps == 8 || warps == 16) ? warps : 0; }
 
 int dasp_denormalize(const float* p01, const float* lo, const float* span, float* out, int* flag, int64_t rows,
                      int64_t cols, void* stream) {
@@ -80,10 +75,6 @@ int dasp_denormalize(const float* p01, const float* lo, const float* span, float
   return DASP_OK;
 }
 
-void dasp_debug_eq_bwd_stages(int stages) { dasp::g_eq_bwd_stages = (stages == 1 || stages == 2) ? stages : 0; }
-
 void dasp_debug_reverb_flat_filterbank(int on) { dasp::g_flat_fb = on ? 1 : 0; }
-
-void dasp_debug_reverb_path(int path) { dasp::g_reverb_path = (path == 1 || path == 2) ? path : 0; }
 
 }  // extern "C"

@@ -47,17 +47,13 @@
 // The 30 sums per row are reduced deterministically; a second tiny kernel adds the channels of an item and applies
 // the fp64 Jacobian d(sg,q,be1,B2,b0)/d(gain_dB, fc, Q) (forward-mode dual numbers).
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
 namespace dasp {
 namespace {
 
-#ifndef DASP_EQ_E
-#define DASP_EQ_E 15
-#endif
-constexpr int kE = DASP_EQ_E;    // samples per lane per tile (odd: conflict-free stride-E shared-memory access)
+constexpr int kE = 15;           // samples per lane per tile (odd: conflict-free stride-E shared-memory access)
 static_assert(kE % 2 == 1, "E must be odd");
 constexpr int kTile = 32 * kE;   // samples per tile (one warp)
 constexpr int kSections = 6;
@@ -145,22 +141,14 @@ __device__ inline M2d mpow(double sg, double q, unsigned n) {
 }
 
 // ------------------------------------------------------------------ arithmetic on row pairs (x = row A, y = row B)
-// DASP_EQ_PACKED = 1 (default) issues Blackwell's packed FFMA2/FMUL2/FADD2 where both operands are row pairs; 0 issues
-// two scalar instructions per pair.  Measured on B200 (profiles/r02_ffma2_probe.md, profiles/r02_eq_variants.md): in a
-// micro-benchmark an FFMA2 with three distinct register-pair operands occupies the FMA pipe ~4.3 cycles per warp
-// (two scalar FFMAs: ~2.4), but inside these kernels the packed form still wins (forward 0.39 vs 0.45 ms): operand
-// reuse between neighbouring instructions is high and the halved issue count matters more.
-#ifndef DASP_EQ_PACKED
-#define DASP_EQ_PACKED 1
-#endif
+// Blackwell's packed FFMA2/FMUL2/FADD2 where both operands are row pairs.  Measured on B200
+// (profiles/r02_ffma2_probe.md, profiles/r02_eq_variants.md): in a micro-benchmark an FFMA2 with three distinct
+// register-pair operands occupies the FMA pipe ~4.3 cycles per warp (two scalar FFMAs: ~2.4), but inside these kernels
+// the packed form still wins over two scalar instructions per pair (forward 0.39 vs 0.45 ms): operand reuse between
+// neighbouring instructions is high and the halved issue count matters more.
 typedef float2 f2;
-#if DASP_EQ_PACKED
 __device__ __forceinline__ f2 ffma2(f2 a, f2 b, f2 c) { return __ffma2_rn(a, b, c); }
 __device__ __forceinline__ f2 fmul2(f2 a, f2 b) { return __fmul2_rn(a, b); }
-#else
-__device__ __forceinline__ f2 ffma2(f2 a, f2 b, f2 c) { return make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y)); }
-__device__ __forceinline__ f2 fmul2(f2 a, f2 b) { return make_float2(a.x * b.x, a.y * b.y); }
-#endif
 __device__ __forceinline__ f2 zero2() { return make_float2(0.f, 0.f); }
 __device__ __forceinline__ f2 shfl_up2(f2 v, int d) {
   return make_float2(__shfl_up_sync(0xffffffffu, v.x, d), __shfl_up_sync(0xffffffffu, v.y, d));
@@ -377,7 +365,6 @@ __device__ __forceinline__ void scan_rev(St& v, const Tables<C>& tb, int k, cons
 // ------------------------------------------------------------------ carry mailboxes between the warps of a CTA
 // mailbox (k, w): carry of section k entering the next tile of warp w; written by the warp of the preceding tile.
 // Use number u of a mailbox completes phase u of its mbarrier (tile/sequence 0 is pre-arrived with a zero carry).
-// With W == 1 the same mailboxes carry the state from one tile to the next of the single warp (__syncwarp only).
 template <int W>
 struct Mail {
   float4* data;     // [kSections][W]
@@ -387,11 +374,11 @@ struct Mail {
     fence_barrier_init();
     for (int k = 0; k < kSections; ++k) {
       data[k * W + 0] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (W > 1) mbar_arrive(&bar[k * W + 0]);
+      mbar_arrive(&bar[k * W + 0]);
     }
   }
   __device__ __forceinline__ St take(int k, int w, int use) {
-    if (W > 1) mbar_wait(&bar[k * W + w], (uint32_t)(use & 1));
+    mbar_wait(&bar[k * W + w], (uint32_t)(use & 1));
     const float4 d = data[k * W + w];
     __syncwarp();                                    // every lane has its copy before the refill may be triggered
     return {make_float2(d.x, d.y), make_float2(d.z, d.w)};
@@ -399,7 +386,7 @@ struct Mail {
   // called by ONE lane (the one that holds the tile total)
   __device__ __forceinline__ void put(int k, int w, const St& c) {
     data[k * W + w] = make_float4(c.s1.x, c.s1.y, c.s2.x, c.s2.y);
-    if (W > 1) mbar_arrive(&bar[k * W + w]);
+    mbar_arrive(&bar[k * W + w]);
   }
 };
 
@@ -480,11 +467,14 @@ __device__ __forceinline__ PairRows pair_rows(int64_t pair, int64_t rows) {
 }
 
 // =============================================================================== forward
-template <class C, int W, int S>
+// per-warp shared memory: two units, double buffered (tile i+W loads while tile i is computed), one barrier each
+template <class C, int W>
+using FwdSmem = Smem<C, W, 2, 2>;
+
+template <class C, int W>
 __global__ void __launch_bounds__(W * 32) eq_fwd_kernel(EqParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  using SM = Smem<C, W, S, S>;
-  SM sm(smem_raw);
+  FwdSmem<C, W> sm(smem_raw);
   const Tables<C>& tb = *sm.tb;
   const int lane = threadIdx.x & 31;
   // the warp index, read from lane 0: the compiler then KNOWS it is warp-uniform.  With `threadIdx.x >> 5` the
@@ -497,7 +487,7 @@ __global__ void __launch_bounds__(W * 32) eq_fwd_kernel(EqParams p) {
   build_tables(*sm.tb, p.params, pr.row_a / p.chs, pr.row_b / p.chs, p.sample_rate);
   Mail<W> mail{sm.mail_data, sm.mail_bar};
   if (threadIdx.x == 0) {
-    for (int i = 0; i < S * W; ++i) mbar_init(&sm.full[i], 1);
+    for (int i = 0; i < 2 * W; ++i) mbar_init(&sm.full[i], 1);
     mail.init_all();
   }
   __syncthreads();
@@ -507,28 +497,22 @@ __global__ void __launch_bounds__(W * 32) eq_fwd_kernel(EqParams p) {
   const float* xb = p.x + pr.row_b * p.n;
   float* ya = p.y + pr.row_a * p.n;
   float* yb = p.y + pr.row_b * p.n;
-  float* my_units = sm.units + (size_t)warp * S * kUnitFloats;
-  uint64_t* my_full = sm.full + warp * S;
+  float* my_units = sm.units + (size_t)warp * 2 * kUnitFloats;
+  uint64_t* my_full = sm.full + warp * 2;
   const StepOffsets so = fwd_offsets(lane);
   float4* ckpt = p.ckpt ? reinterpret_cast<float4*>(p.ckpt) + (int64_t)blockIdx.x * p.ntiles * kSections : nullptr;
 
-  if (S > 1 && warp < p.ntiles) warp_load(my_units, xa, xb, warp, rp, &my_full[0], lane);
+  if (warp < p.ntiles) warp_load(my_units, xa, xb, warp, rp, &my_full[0], lane);
   int jt = 0;
   for (int i = warp; i < p.ntiles; i += W, ++jt) {
-    const int st = (S > 1) ? (jt & 1) : 0;
+    const int st = jt & 1;
     float* unit = my_units + (size_t)st * kUnitFloats;
-    if (S > 1) {
-      if (i + W < p.ntiles) {
-        // the other stage was stored from one tile ago: that bulk store must have finished READING it
-        if (rp.bulk && lane == 0) tma_store_wait_read<0>();
-        warp_load(my_units + (size_t)(st ^ 1) * kUnitFloats, xa, xb, i + W, rp, &my_full[st ^ 1], lane);
-      }
-    } else {
+    if (i + W < p.ntiles) {
+      // the other stage was stored from one tile ago: that bulk store must have finished READING it
       if (rp.bulk && lane == 0) tma_store_wait_read<0>();
-      __syncwarp();
-      warp_load(unit, xa, xb, i, rp, &my_full[0], lane);
+      warp_load(my_units + (size_t)(st ^ 1) * kUnitFloats, xa, xb, i + W, rp, &my_full[st ^ 1], lane);
     }
-    if (rp.bulk) mbar_wait(&my_full[st], (uint32_t)(((S > 1) ? (jt >> 1) : jt) & 1));
+    if (rp.bulk) mbar_wait(&my_full[st], (uint32_t)((jt >> 1) & 1));
     const int off = lane * kE;
     const int64_t n0 = (int64_t)i * kTile + off;
     f2 v[kE];
@@ -562,16 +546,20 @@ __global__ void __launch_bounds__(W * 32) eq_fwd_kernel(EqParams p) {
 }
 
 // =============================================================================== backward
-// per-warp shared memory: X[S], G[S] (row-pair units, TMA) and U1..U4 (interleaved f2, the inputs of sections 1..4);
-// the input of section 5 overwrites the G unit once dL/dy sits in registers, and dL/dx leaves through the G unit.
-template <int S>
-struct BwdUnits { static constexpr int kPerWarp = 2 * S + 4; };
+// Warps per row pair.  The backward holds 255 registers per thread, i.e. 8 warps per SM whatever the split: W=8 with
+// one load stage (one CTA per SM, least shared memory per warp) measured best on B200 (profiles/r02_eq_variants.md).
+constexpr int kBwdWarps = 8;
+// per-warp shared memory: the x and dL/dy units (row-pair units, TMA, one barrier) and U1..U4 (interleaved f2, the
+// inputs of sections 1..4); the input of section 5 overwrites the dL/dy unit once dL/dy sits in registers, and dL/dx
+// leaves through the same unit.
+template <class C>
+using BwdSmem = Smem<C, kBwdWarps, 6, 1>;
 
-template <class C, int W, int S>
-__global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
+template <class C>
+__global__ void __launch_bounds__(kBwdWarps * 32) eq_bwd_kernel(EqParams p) {
+  constexpr int W = kBwdWarps;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  using SM = Smem<C, W, BwdUnits<S>::kPerWarp, S>;
-  SM sm(smem_raw);
+  BwdSmem<C> sm(smem_raw);
   const Tables<C>& tb = *sm.tb;
   __shared__ double red[W][kSections * 5][2];
   const int lane = threadIdx.x & 31;
@@ -587,7 +575,7 @@ __global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
   build_tables(*sm.tb, p.params, row_a / p.chs, row_b / p.chs, p.sample_rate);
   Mail<W> mail{sm.mail_data, sm.mail_bar};
   if (threadIdx.x == 0) {
-    for (int i = 0; i < S * W; ++i) mbar_init(&sm.full[i], 1);
+    for (int i = 0; i < W; ++i) mbar_init(&sm.full[i], 1);
     mail.init_all();
   }
   __syncthreads();
@@ -599,11 +587,11 @@ __global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
   const float* gb = p.gy + row_b * p.n;
   float* oa = p.y + row_a * p.n;
   float* ob = p.y + row_b * p.n;
-  float* my = sm.units + (size_t)warp * BwdUnits<S>::kPerWarp * kUnitFloats;
-  float* X = my;                                   // [S] units
-  float* G = my + (size_t)S * kUnitFloats;         // [S] units
-  f2* U = reinterpret_cast<f2*>(my + (size_t)2 * S * kUnitFloats);     // [4][kTile] f2: inputs of sections 1..4
-  uint64_t* my_full = sm.full + warp * S;
+  float* my = sm.units + (size_t)warp * 6 * kUnitFloats;
+  float* xu = my;                                  // x unit
+  float* gu = my + kUnitFloats;                    // dL/dy unit, then the input of section 5, then dL/dx
+  f2* U = reinterpret_cast<f2*>(my + (size_t)2 * kUnitFloats);     // [4][kTile] f2: inputs of sections 1..4
+  uint64_t* full = sm.full + warp;
   const StepOffsets so_f = fwd_offsets(lane), so_r = rev_offsets(lane);
   const float4* ckpt = reinterpret_cast<const float4*>(p.ckpt) + (int64_t)blockIdx.x * p.ntiles * kSections;
 
@@ -614,47 +602,31 @@ __global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
     for (int q = 0; q < 5; ++q) acc[k][q] = zero2();
   }
 
-  auto load_seq = [&](int seq, int stage) {        // x and dL/dy tiles of sequence number seq complete on ONE barrier
-    const int tile = p.ntiles - 1 - seq;
-    const int64_t pos = (int64_t)tile * kTile;
-    const int len = rp.len_of(tile);
-    float* xu = X + (size_t)stage * kUnitFloats;
-    float* gu = G + (size_t)stage * kUnitFloats;
-    if (rp.bulk) {
-      if (lane == 0) {
-        mbar_arrive_expect_tx(&my_full[stage], (uint32_t)len * 16u);
-        tma_load_1d(xu, xa + pos, (uint32_t)len * 4u, &my_full[stage]);
-        tma_load_1d(xu + kTile, xb + pos, (uint32_t)len * 4u, &my_full[stage]);
-        tma_load_1d(gu, ga + pos, (uint32_t)len * 4u, &my_full[stage]);
-        tma_load_1d(gu + kTile, gb + pos, (uint32_t)len * 4u, &my_full[stage]);
-      }
-    } else {
-      for (int i = lane; i < len; i += 32) {
-        xu[i] = xa[pos + i]; xu[kTile + i] = xb[pos + i];
-        gu[i] = ga[pos + i]; gu[kTile + i] = gb[pos + i];
-      }
-      __syncwarp();
-    }
-  };
-
-  if (S > 1 && warp < p.ntiles) load_seq(warp, 0);
   int jt = 0;
   for (int seq = warp; seq < p.ntiles; seq += W, ++jt) {
-    const int st = (S > 1) ? (jt & 1) : 0;
     const int tile = p.ntiles - 1 - seq;
-    if (S > 1) {
-      if (seq + W < p.ntiles) {
-        if (rp.bulk && lane == 0) tma_store_wait_read<0>();      // the store that left from G[st ^ 1] one tile ago
-        load_seq(seq + W, st ^ 1);
+    if (rp.bulk && lane == 0) tma_store_wait_read<0>();      // the store of the previous tile has finished reading gu
+    __syncwarp();
+    {  // x and dL/dy tiles complete on ONE barrier
+      const int64_t pos = (int64_t)tile * kTile;
+      const int len = rp.len_of(tile);
+      if (rp.bulk) {
+        if (lane == 0) {
+          mbar_arrive_expect_tx(full, (uint32_t)len * 16u);
+          tma_load_1d(xu, xa + pos, (uint32_t)len * 4u, full);
+          tma_load_1d(xu + kTile, xb + pos, (uint32_t)len * 4u, full);
+          tma_load_1d(gu, ga + pos, (uint32_t)len * 4u, full);
+          tma_load_1d(gu + kTile, gb + pos, (uint32_t)len * 4u, full);
+        }
+      } else {
+        for (int i = lane; i < len; i += 32) {
+          xu[i] = xa[pos + i]; xu[kTile + i] = xb[pos + i];
+          gu[i] = ga[pos + i]; gu[kTile + i] = gb[pos + i];
+        }
+        __syncwarp();
       }
-    } else {
-      if (rp.bulk && lane == 0) tma_store_wait_read<0>();
-      __syncwarp();
-      load_seq(seq, 0);
     }
-    if (rp.bulk) mbar_wait(&my_full[st], (uint32_t)(((S > 1) ? (jt >> 1) : jt) & 1));
-    const float* xu = X + (size_t)st * kUnitFloats;
-    float* gu = G + (size_t)st * kUnitFloats;
+    if (rp.bulk) mbar_wait(full, (uint32_t)(jt & 1));
     f2* U5 = reinterpret_cast<f2*>(gu);            // input of section 5, interleaved, over the consumed dL/dy unit
     const int off = lane * kE;
     const int64_t n0 = (int64_t)tile * kTile + off;
@@ -765,7 +737,7 @@ __global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
           l1 = t1;
         }
       }
-      if (k == kSections - 1) __syncwarp();        // every lane has read its u_5 before dL/dx may land in the G unit
+      if (k == kSections - 1) __syncwarp();        // every lane has read its u_5 before dL/dx may land in the dL/dy unit
     }
 #pragma unroll
     for (int j = 0; j < kE; ++j) { gu[off + j] = gq[j].x; gu[kTile + off + j] = gq[j].y; }
@@ -783,7 +755,7 @@ __global__ void __launch_bounds__(W * 32) eq_bwd_kernel(EqParams p) {
     }
   }
   __syncthreads();
-  for (int o = threadIdx.x; o < kSections * 5 * 2; o += W * 32) {      // W = 1 has fewer threads than outputs
+  for (int o = threadIdx.x; o < kSections * 5 * 2; o += W * 32) {
     const int h = o / (kSections * 5), e = o - h * (kSections * 5);
     double s = 0.0;
 #pragma unroll
@@ -818,40 +790,16 @@ __global__ void eq_param_grad_kernel(const float* __restrict__ partial, const fl
 }
 
 // ---- host side -----------------------------------------------------------------------------
-// experiment knobs (read once): DASP_EQ_FWD_W / DASP_EQ_BWD_W = warps per row pair, DASP_EQ_FWD_S / DASP_EQ_BWD_S =
-// load stages per warp.  0 / unset = automatic.
-int env_int(const char* name) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : 0;
-}
-int tune_fwd_w() { static const int v = env_int("DASP_EQ_FWD_W"); return v; }
-int tune_fwd_s() { static const int v = env_int("DASP_EQ_FWD_S"); return v; }
-int tune_bwd_w() { static const int v = env_int("DASP_EQ_BWD_W"); return v; }
-int tune_bwd_s() {
-  static const int v = env_int("DASP_EQ_BWD_S");
-  return debug_eq_bwd_stages() ? debug_eq_bwd_stages() : v;
-}
-// force the general (pair-coefficient) tables even when every pair lies inside one item: test hook via the env
-int tune_force_pair_tables() { static const int v = env_int("DASP_EQ_PAIR_TABLES"); return v; }
-
-// Warps per row pair (W in {1, 2, 3, 4, 8}, forward also 16; 0 / other = automatic).  Measured on B200 at 1024 pairs x 48000 samples
-// (profiles/r02_eq_variants.md): forward W=4 with two load stages beats W=2 and the single-wave choices; small batches
-// want W=8 to fill the SMs at all.  The backward holds 255 registers per thread, i.e. 8 warps per SM whatever the
-// split: W=8 with one stage (one CTA per SM, least shared memory per warp) measured best.
-bool valid_w(int w) { return w == 1 || w == 2 || w == 3 || w == 4 || w == 8; }
-// The forward also has W = 16 (512 threads, 80 registers): when there is at most one row pair per SM (e.g. 1024 stereo
-// items split over 8 GPUs) a pair's CTA is alone on its SM, and sixteen warps walk its tiles twice as fast as eight.
-// The backward cannot follow (255 registers per thread x 512 threads exceed the register file).
-int pick_fwd_warps(int64_t pairs, int tuned) {
-  const int f = debug_forced_warps() ? debug_forced_warps() : tuned;
-  if (valid_w(f) || f == 16) return f;
+// Warps per row pair of the forward (dasp_debug_force_warps pins 4, 8 or 16).  Measured on B200 at 1024 pairs x 48000
+// samples (profiles/r02_eq_variants.md): W=4 with two load stages beats W=2 and the single-wave choices; small batches
+// want W=8 to fill the SMs at all.  W = 16 (512 threads, 80 registers): when there is at most one row pair per SM
+// (e.g. 1024 stereo items split over 8 GPUs) a pair's CTA is alone on its SM, and sixteen warps walk its tiles twice as
+// fast as eight.  The backward cannot follow (255 registers per thread x 512 threads exceed the register file).
+int pick_fwd_warps(int64_t pairs) {
+  const int f = debug_forced_warps();
+  if (f == 4 || f == 8 || f == 16) return f;
   if (pairs <= sm_count()) return 16;
   return (pairs * 4 < 20ll * sm_count()) ? 8 : 4;
-}
-int pick_bwd_warps(int tuned) {
-  const int f = debug_forced_warps() ? debug_forced_warps() : tuned;
-  if (valid_w(f)) return f;
-  return 8;
 }
 
 // one-off opt-in to > 48 KB dynamic shared memory, cached per (host thread, device, kernel INSTANTIATION): the
@@ -868,59 +816,32 @@ int ensure_smem(size_t bytes) {
   return DASP_OK;
 }
 
-template <class C, int W, int S>
+template <class C, int W>
 int launch_fwd(const EqParams& p, int64_t pairs, cudaStream_t st) {
-  constexpr size_t smem = Smem<C, W, S, S>::kBytes;
-  if constexpr (smem <= kSmemPerSm) {
-    int rc = ensure_smem<eq_fwd_kernel<C, W, S>>(smem);
-    if (rc != DASP_OK) return rc;
-    eq_fwd_kernel<C, W, S><<<(unsigned)pairs, W * 32, smem, st>>>(p);
-    DASP_LAUNCH_OK("eq_fwd_kernel");
-    return DASP_OK;
-  } else {
-    set_error("eq fwd: variant W=%d S=%d needs %zu bytes of shared memory", W, S, smem);
-    return DASP_ERR_INVALID;
-  }
-}
-template <class C, int W, int S>
-int launch_bwd(const EqParams& p, int64_t pairs, cudaStream_t st) {
-  constexpr size_t smem = Smem<C, W, BwdUnits<S>::kPerWarp, S>::kBytes;
-  if constexpr (smem <= kSmemPerSm) {
-    int rc = ensure_smem<eq_bwd_kernel<C, W, S>>(smem);
-    if (rc != DASP_OK) return rc;
-    eq_bwd_kernel<C, W, S><<<(unsigned)pairs, W * 32, smem, st>>>(p);
-    DASP_LAUNCH_OK("eq_bwd_kernel");
-    return DASP_OK;
-  } else {
-    set_error("eq bwd: variant W=%d S=%d needs %zu bytes of shared memory (E=%d)", W, S, smem, kE);
-    return DASP_ERR_INVALID;
-  }
-}
-template <class C, int S>
-int dispatch_fwd(int w, const EqParams& p, int64_t pairs, cudaStream_t st) {
-  switch (w) {
-    case 1: return launch_fwd<C, 1, S>(p, pairs, st);
-    case 2: return launch_fwd<C, 2, S>(p, pairs, st);
-    case 3: return launch_fwd<C, 3, S>(p, pairs, st);
-    case 4: return launch_fwd<C, 4, S>(p, pairs, st);
-    case 16: return launch_fwd<C, 16, S>(p, pairs, st);
-    default: return launch_fwd<C, 8, S>(p, pairs, st);
-  }
+  constexpr size_t smem = FwdSmem<C, W>::kBytes;
+  static_assert(smem <= kSmemPerSm, "eq fwd: shared memory of one CTA exceeds the SM");
+  int rc = ensure_smem<eq_fwd_kernel<C, W>>(smem);
+  if (rc != DASP_OK) return rc;
+  eq_fwd_kernel<C, W><<<(unsigned)pairs, W * 32, smem, st>>>(p);
+  DASP_LAUNCH_OK("eq_fwd_kernel");
+  return DASP_OK;
 }
 template <class C>
-int dispatch_bwd(int w, int stages, const EqParams& p, int64_t pairs, cudaStream_t st) {
-  switch (w * 10 + stages) {
-    case 11: return launch_bwd<C, 1, 1>(p, pairs, st);
-    case 12: return launch_bwd<C, 1, 2>(p, pairs, st);
-    case 21: return launch_bwd<C, 2, 1>(p, pairs, st);
-    case 22: return launch_bwd<C, 2, 2>(p, pairs, st);
-    case 31: return launch_bwd<C, 3, 1>(p, pairs, st);
-    case 32: return launch_bwd<C, 3, 2>(p, pairs, st);
-    case 41: return launch_bwd<C, 4, 1>(p, pairs, st);
-    case 42: return launch_bwd<C, 4, 2>(p, pairs, st);
-    case 82: if constexpr (Smem<C, 8, BwdUnits<2>::kPerWarp, 2>::kBytes <= kSmemPerSm) return launch_bwd<C, 8, 2>(p, pairs, st);
-             [[fallthrough]];
-    default: return launch_bwd<C, 8, 1>(p, pairs, st);
+int launch_bwd(const EqParams& p, int64_t pairs, cudaStream_t st) {
+  constexpr size_t smem = BwdSmem<C>::kBytes;
+  static_assert(smem <= kSmemPerSm, "eq bwd: shared memory of one CTA exceeds the SM");
+  int rc = ensure_smem<eq_bwd_kernel<C>>(smem);
+  if (rc != DASP_OK) return rc;
+  eq_bwd_kernel<C><<<(unsigned)pairs, kBwdWarps * 32, smem, st>>>(p);
+  DASP_LAUNCH_OK("eq_bwd_kernel");
+  return DASP_OK;
+}
+template <class C>
+int dispatch_fwd(int w, const EqParams& p, int64_t pairs, cudaStream_t st) {
+  switch (w) {
+    case 4: return launch_fwd<C, 4>(p, pairs, st);
+    case 16: return launch_fwd<C, 16>(p, pairs, st);
+    default: return launch_fwd<C, 8>(p, pairs, st);
   }
 }
 
@@ -947,16 +868,14 @@ int dasp_eq_fwd(const float* x, const float* params, float* y, float* ckpt, int6
   DASP_REQUIRE(sample_rate > 0.f, "eq fwd: sample_rate must be positive");
   const int64_t rows = bs * chs, pairs = (rows + 1) / 2;
   DASP_REQUIRE(pairs < (1ll << 31), "eq fwd: too many rows");
-  const int stages = tune_fwd_s() == 1 ? 1 : 2;
-  const int w = pick_fwd_warps(pairs, tune_fwd_w());
+  const int w = pick_fwd_warps(pairs);
   EqParams p{};
   p.x = x; p.y = y; p.params = params; p.ckpt = ckpt; p.n = n; p.rows = rows; p.chs = (int)chs;
   p.ntiles = (int)((n + kTile - 1) / kTile); p.sample_rate = sample_rate;
   p.bulk = (n % 4 == 0) && aligned16(x) && aligned16(y);
   cudaStream_t st = (cudaStream_t)stream;
-  const bool same_item = (chs % 2 == 0) && !tune_force_pair_tables();      // rows 2p and 2p+1 share their item
-  if (same_item) return stages == 1 ? dispatch_fwd<float, 1>(w, p, pairs, st) : dispatch_fwd<float, 2>(w, p, pairs, st);
-  return stages == 1 ? dispatch_fwd<f2, 1>(w, p, pairs, st) : dispatch_fwd<f2, 2>(w, p, pairs, st);
+  const bool same_item = chs % 2 == 0;      // rows 2p and 2p+1 share their item
+  return same_item ? dispatch_fwd<float>(w, p, pairs, st) : dispatch_fwd<f2>(w, p, pairs, st);
 }
 
 int dasp_eq_bwd(const float* gy, const float* x, const float* params, const float* ckpt, float* gx,
@@ -975,14 +894,11 @@ int dasp_eq_bwd(const float* gy, const float* x, const float* params, const floa
     set_error("eq bwd: workspace needs %lld floats, got %lld", (long long)(rows * 30), (long long)ws_floats);
     return DASP_ERR_WORKSPACE;
   }
-  const int stages = tune_bwd_s() == 2 ? 2 : 1;
-  const int w = pick_bwd_warps(tune_bwd_w());
   EqParams p{};
   p.x = x; p.gy = gy; p.y = gx; p.params = params; p.ckpt = const_cast<float*>(ckpt); p.partial = ws; p.n = n;
   p.rows = rows; p.chs = (int)chs; p.ntiles = (int)((n + kTile - 1) / kTile); p.sample_rate = sample_rate;
   p.bulk = (n % 4 == 0) && aligned16(x) && aligned16(gy) && aligned16(gx);
-  const bool same_item = (chs % 2 == 0) && !tune_force_pair_tables();
-  const int rc = same_item ? dispatch_bwd<float>(w, stages, p, pairs, st) : dispatch_bwd<f2>(w, stages, p, pairs, st);
+  const int rc = chs % 2 == 0 ? launch_bwd<float>(p, pairs, st) : launch_bwd<f2>(p, pairs, st);
   if (rc != DASP_OK) return rc;
   const int64_t tot = bs * kSections;
   eq_param_grad_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(ws, params, gparams, bs, (int)chs, sample_rate);

@@ -55,15 +55,10 @@ static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t
 
 int sm_count();  // cached cudaDevAttrMultiProcessorCount of the current device
 
-// Test hook (dasp_debug_force_warps): 0 = automatic; 1/2/3/4/8/16 pins the warps-per-row choice of the scan kernels
-// (a kernel family that has no such variant keeps its automatic choice)
-// so that every kernel variant can be exercised at small, cheap-to-check batch sizes.
+// Test hook (dasp_debug_force_warps): 0 = automatic; 1/2/4/8/16 pins the warps-per-row choice of the scan kernels
+// (the EQ forward has 4/8/16, the compressor all five; a kernel family that has no such variant keeps its automatic
+// choice) so that every kernel variant can be exercised at small, cheap-to-check batch sizes.
 int debug_forced_warps();
-// Test hook (dasp_debug_eq_bwd_stages): 0 = automatic; 1 / 2 pins the number of x / dL/dy stages of the EQ backward
-int debug_eq_bwd_stages();
-// Test hook (dasp_debug_reverb_path): IR synthesis of the device-noise reverb: 0 = automatic, 1 = generator / cuFFT /
-// shaping kernels, 2 = single cluster kernel
-int debug_reverb_path();
 // Test hook (dasp_debug_reverb_flat_filterbank): the spectral IR synthesis uses unit-impulse "filters", so the
 // band-filtered noise it keeps for the backward IS the periodic white sequence w_k the generator draws; the parity
 // test rebuilds the reference-style noise tensor from it and checks the default path against the oracle.

@@ -19,7 +19,6 @@
 // w[n] = ds[n] + a w[n+1] with the mirrored scan (shfl_down), accumulates the five parameter
 // gradients in registers across tiles (deterministic), and writes dL/dx in place.
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tile_pipe.cuh"
@@ -27,17 +26,9 @@
 namespace dasp {
 namespace {
 
-#ifndef DASP_DYN_E
-#define DASP_DYN_E 7
-#endif
-constexpr int kE = DASP_DYN_E;        // samples per thread per tile; odd => stride-E smem access is conflict-free
-#ifndef DASP_DYN_STAGES
-#define DASP_DYN_STAGES 3
-#endif
-#ifndef DASP_DYN_BWD_MINB
-#define DASP_DYN_BWD_MINB 4      // resident CTAs per SM the backward is compiled for at W = 4 (register budget 65536 / (128 * MINB))
-#endif
-constexpr int kStages = DASP_DYN_STAGES;
+constexpr int kE = 7;                 // samples per thread per tile; odd => stride-E smem access is conflict-free
+constexpr int kStages = 3;
+constexpr int kBwdMinBlocks = 4;      // resident CTAs per SM the backward is compiled for at W = 4 (register budget 65536 / (128 * 4))
 constexpr int kMaxChs = 32;
 constexpr float kDbPerLog2 = 6.020599913279624f;    // 20*log10(2)
 constexpr float kDbGradScale = 8.685889638065035f;  // 20/ln(10)
@@ -356,7 +347,7 @@ __global__ void __launch_bounds__(W * 32) dynamics_fwd_kernel(DynParams p) {
 
 // =============================================================================== backward
 template <Curve CV, int W, bool LA, bool ST = false>
-__global__ void __launch_bounds__(W * 32, (W <= 4) ? (4 * DASP_DYN_BWD_MINB) / W : (W == 8 ? 2 : 1)) dynamics_bwd_kernel(DynParams p) {
+__global__ void __launch_bounds__(W * 32, (W <= 4) ? (4 * kBwdMinBlocks) / W : (W == 8 ? 2 : 1)) dynamics_bwd_kernel(DynParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   Smem<W> sm(smem_raw);
   __shared__ float red[5][W];
@@ -568,12 +559,6 @@ int pick_warps(int64_t bs, int chs, int nbuf_per_ch) {
   while (w > 1 && !fits(w)) w /= 2;
   return w;
 }
-// experiment / test knob: DASP_DYN_GENERIC=1 disables the stereo specialisation (the generic channel loop is the path
-// every other channel count takes, so the two are compared on the same stereo inputs by the tests)
-int debug_generic_channels() {
-  const char* v = getenv("DASP_DYN_GENERIC");
-  return (v && atoi(v)) ? 1 : 0;
-}
 
 // one-off opt-in to the largest dynamic shared memory any launch of `kernel` may ask for (pick_warps caps it at
 // 96 KB / 200 KB), cached per (host thread, device, kernel instantiation: a non-type template parameter) instead of a driver call on every launch
@@ -609,14 +594,12 @@ int launch_bwd_la(const DynParams& p, int64_t bs, cudaStream_t st) {
 template <Curve CV, int W>
 int launch_fwd_w(const DynParams& p, int64_t bs, cudaStream_t st) {
   if (p.lookahead > 0) return launch_fwd_la<CV, W, true, false>(p, bs, st);
-  return (p.chs == 2 && !debug_generic_channels()) ? launch_fwd_la<CV, W, false, true>(p, bs, st)
-                                                   : launch_fwd_la<CV, W, false, false>(p, bs, st);
+  return p.chs == 2 ? launch_fwd_la<CV, W, false, true>(p, bs, st) : launch_fwd_la<CV, W, false, false>(p, bs, st);
 }
 template <Curve CV, int W>
 int launch_bwd_w(const DynParams& p, int64_t bs, cudaStream_t st) {
   if (p.lookahead > 0) return launch_bwd_la<CV, W, true, false>(p, bs, st);
-  return (p.chs == 2 && !debug_generic_channels()) ? launch_bwd_la<CV, W, false, true>(p, bs, st)
-                                                   : launch_bwd_la<CV, W, false, false>(p, bs, st);
+  return p.chs == 2 ? launch_bwd_la<CV, W, false, true>(p, bs, st) : launch_bwd_la<CV, W, false, false>(p, bs, st);
 }
 
 template <Curve CV>

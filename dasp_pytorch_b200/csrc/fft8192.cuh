@@ -43,20 +43,15 @@ constexpr int kPlaneY = 9216;          // floats per plane of the padded buffer 
 constexpr int kTabFloats = 2 * (2 * 64) + 2 * (2 * 512) + 2 * 1024 + 2 * 128;   // see Tables
 
 // ---- packed lane pair ------------------------------------------------------------------------------
-// DASP_FFT_PACKED = 1 (default): the lane pair is one packed fp32x2 register pair (FADD2/FMUL2/FFMA2); 0: the same
-// two lanes as two scalar instructions.  A/B on B200 (profiles/r02_eq_variants.md): although a micro-benchmark shows
-// FFMA2 with three distinct register pairs at half the FMA-pipe throughput of two scalar FFMAs (FADD2 is at parity),
-// the packed FFT kernels are 1-6 % FASTER end to end (reverb forward 6.11 vs 6.47 ms), so packed stays.
-#ifndef DASP_FFT_PACKED
-#define DASP_FFT_PACKED 1
-#endif
-// DASP_FFT_TWIDDLE_RECURRENCE = 1 (default): the seven twiddles a thread needs in a pass are successive powers of one
-// table entry, formed by complex multiplication in registers instead of being fetched one by one -- the FFT kernels are
-// bound by the shared-memory pipe (data exchange + twiddle fetches), not by the FMA pipe (profiles/r02_reverb_*.md).
-#ifndef DASP_FFT_TWIDDLE_RECURRENCE
-#define DASP_FFT_TWIDDLE_RECURRENCE 1
-#endif
-#if defined(__CUDA_ARCH__) && DASP_FFT_PACKED
+// On the device the lane pair is one packed fp32x2 register pair (FADD2/FMUL2/FFMA2).  A/B on B200
+// (profiles/r02_eq_variants.md): although a micro-benchmark shows FFMA2 with three distinct register pairs at half the
+// FMA-pipe throughput of two scalar FFMAs (FADD2 is at parity), the packed FFT kernels are 1-6 % FASTER end to end
+// than two scalar instructions per pair (reverb forward 6.11 vs 6.47 ms).  The host emulation keeps two scalars.
+//
+// Twiddles: the seven twiddles a thread needs in a pass are successive powers of one table entry, formed by complex
+// multiplication in registers instead of being fetched one by one -- the FFT kernels are bound by the shared-memory
+// pipe (data exchange + twiddle fetches), not by the FMA pipe (profiles/r02_reverb_*.md).
+#if defined(__CUDA_ARCH__)
 struct V2 { float2 v; };
 DASP_HD V2 v2(float a, float b) { V2 r; r.v = make_float2(a, b); return r; }
 DASP_HD V2 bc(float a) { return v2(a, a); }
@@ -70,20 +65,6 @@ DASP_HD float lane0(V2 a) { return a.v.x; }
 DASP_HD float lane1(V2 a) { return a.v.y; }
 DASP_HD V2 ld2(const float* p) { V2 r; r.v = *reinterpret_cast<const float2*>(p); return r; }
 DASP_HD void st2(float* p, V2 a) { *reinterpret_cast<float2*>(p) = a.v; }
-#elif defined(__CUDA_ARCH__)
-struct V2 { float x, y; };
-DASP_HD V2 v2(float a, float b) { V2 r; r.x = a; r.y = b; return r; }
-DASP_HD V2 bc(float a) { return v2(a, a); }
-DASP_HD V2 operator+(V2 a, V2 b) { return v2(a.x + b.x, a.y + b.y); }
-DASP_HD V2 operator-(V2 a, V2 b) { return v2(a.x - b.x, a.y - b.y); }
-DASP_HD V2 operator*(V2 a, V2 b) { return v2(a.x * b.x, a.y * b.y); }
-DASP_HD V2 fma2(V2 a, V2 b, V2 c) { return v2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y)); }
-DASP_HD V2 fnma2(V2 a, V2 b, V2 c) { return v2(fmaf(-a.x, b.x, c.x), fmaf(-a.y, b.y, c.y)); }
-DASP_HD V2 neg(V2 a) { return v2(-a.x, -a.y); }
-DASP_HD float lane0(V2 a) { return a.x; }
-DASP_HD float lane1(V2 a) { return a.y; }
-DASP_HD V2 ld2(const float* p) { const float2 t = *reinterpret_cast<const float2*>(p); return v2(t.x, t.y); }
-DASP_HD void st2(float* p, V2 a) { *reinterpret_cast<float2*>(p) = make_float2(a.x, a.y); }
 #else
 struct V2 { float x, y; };
 DASP_HD V2 v2(float a, float b) { V2 r; r.x = a; r.y = b; return r; }
@@ -191,7 +172,6 @@ DASP_HD void p1(float* gr, float* gi, const Tables& tb, int t) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) { r[j] = ld2(gr + 1024 * j + m); i[j] = ld2(gi + 1024 * j + m); }
   dft8<INV>(r, i);
-#if DASP_FFT_TWIDDLE_RECURRENCE
   {  // w64^(n2 k1) = (w64^n2)^k1: one table entry, six complex multiplies instead of six more (pairs of) loads
     const V2 w1r = ld2(tb.w64b_c + 2 * n2), w1i = ld2(tb.w64b_s + 2 * n2);
     V2 wr = w1r, wi = w1i;
@@ -201,10 +181,6 @@ DASP_HD void p1(float* gr, float* gi, const Tables& tb, int t) {
       if (k1 < 7) cmul<true>(wr, wi, w1r, w1i);
     }
   }
-#else
-#pragma unroll
-  for (int k1 = 1; k1 < 8; ++k1) cmul<INV>(r[k1], i[k1], ld2(tb.w64b_c + 2 * (n2 * k1)), ld2(tb.w64b_s + 2 * (n2 * k1)));
-#endif
 #pragma unroll
   for (int k1 = 0; k1 < 8; ++k1) { st2(gr + 1024 * k1 + m, r[k1]); st2(gi + 1024 * k1 + m, i[k1]); }
 }
@@ -217,7 +193,6 @@ DASP_HD void p2(const float* gr, const float* gi, float* yr, float* yi, const Ta
 #pragma unroll
   for (int n2 = 0; n2 < 8; ++n2) { r[n2] = ld2(gr + src + 128 * n2); i[n2] = ld2(gi + src + 128 * n2); }
   dft8<INV>(r, i);
-#if DASP_FFT_TWIDDLE_RECURRENCE
   // w512^(n3 (k1 + 8 k2)) = w512^(n3 k1) * (w64^n3)^k2: two table entries and seven complex multiplies
   V2 wr = ld2(tb.w512b_c + 2 * (n3 * k1)), wi = ld2(tb.w512b_s + 2 * (n3 * k1));
   const V2 sr = ld2(tb.w64b_c + 2 * n3), si = ld2(tb.w64b_s + 2 * n3);
@@ -227,14 +202,6 @@ DASP_HD void p2(const float* gr, const float* gi, float* yr, float* yi, const Ta
     st2(yr + dst + 144 * k2, r[k2]); st2(yi + dst + 144 * k2, i[k2]);
     if (k2 < 7) cmul<true>(wr, wi, sr, si);
   }
-#else
-#pragma unroll
-  for (int k2 = 0; k2 < 8; ++k2) {
-    const int e = n3 * (k1 + 8 * k2);
-    cmul<INV>(r[k2], i[k2], ld2(tb.w512b_c + 2 * e), ld2(tb.w512b_s + 2 * e));
-    st2(yr + dst + 144 * k2, r[k2]); st2(yi + dst + 144 * k2, i[k2]);
-  }
-#endif
 }
 
 struct P3Regs { V2 r[8], i[8]; };
@@ -252,8 +219,8 @@ DASP_HD void p3_store(float* yr, float* yi, const Tables& tb, int t, P3Regs& q) 
   dft8<INV>(q.r, q.i);
   const int qq = k1 + 8 * k2, n4a = 2 * j, n4b = 2 * j + 1;
   const V2 bwr = v2(tb.w8k_c[n4a * qq], tb.w8k_c[n4b * qq]), bwi = v2(tb.w8k_s[n4a * qq], tb.w8k_s[n4b * qq]);
-#if DASP_FFT_TWIDDLE_RECURRENCE
-  // w8192^(n4 (qq + 64 k3)) = w8192^(n4 qq) * (w128^n4)^k3: the same multiply count as before, 24 fewer scalar loads
+  // w8192^(n4 (qq + 64 k3)) = w8192^(n4 qq) * (w128^n4)^k3: no more multiplies than a per-k3 table lookup needs,
+  // 24 fewer scalar loads
   const V2 sr = v2(tb.w128_c[n4a], tb.w128_c[n4b]), si = v2(tb.w128_s[n4a], tb.w128_s[n4b]);
   V2 wr = bwr, wi = bwi;
 #pragma unroll
@@ -263,19 +230,6 @@ DASP_HD void p3_store(float* yr, float* yi, const Tables& tb, int t, P3Regs& q) 
     st2(yr + dst, q.r[k3]); st2(yi + dst, q.i[k3]);
     if (k3 < 7) cmul<true>(wr, wi, sr, si);
   }
-#else
-#pragma unroll
-  for (int k3 = 0; k3 < 8; ++k3) {
-    V2 wr = bwr, wi = bwi;
-    if (k3 > 0) {
-      const V2 sr = v2(tb.w128_c[n4a * k3], tb.w128_c[n4b * k3]), si = v2(tb.w128_s[n4a * k3], tb.w128_s[n4b * k3]);
-      cmul<true>(wr, wi, sr, si);
-    }
-    cmul<INV>(q.r[k3], q.i[k3], wr, wi);
-    const int dst = 18 * (qq + 64 * k3) + 2 * j;
-    st2(yr + dst, q.r[k3]); st2(yi + dst, q.i[k3]);
-  }
-#endif
 }
 
 // out_r[k4], out_i[k4] = X[t + 512 k4]

@@ -15,7 +15,9 @@
 //   * IR synthesis, device noise (default): spectral_gen_kernel draws the FILTERED noise spectrum directly
 //     (Philox4x32-10 + Box-Muller; see the comment at the kernel); ifft_shape_kernel = own in-shared-memory inverse
 //     FFT (fft8192.cuh) fused with envelope * gain * band mean -> IR written straight into the partition layout of
-//     the convolution.  (Test-hook variants: batched cuFFT + shape_ir_pp_kernel, and one cluster kernel per item.)
+//     the convolution.  Filter banks of 2047 taps or more (transform length nb > 8192) take batched cuFFT +
+//     shape_ir_pp_kernel instead; polyphase factors R > 16 take the overlap-save path of parity mode, fed by
+//     time-domain Philox noise.
 //   * IR synthesis, parity mode (caller's noise tensor): overlap-save blocks -> C2C -> cmul_filter_pairs ->
 //     inverse C2C -> shape_ir_pairs_kernel.
 //   * Audio convolution: uniformly partitioned overlap-save in the frequency domain: x_fft_kernel (window gather +
@@ -225,14 +227,9 @@ __global__ void cmul_filter_pairs_kernel(float2* __restrict__ C, const float2* _
   }
 }
 
-// packed fp32x2 helpers of the generator's R-point DFT: scalar pairs unless DASP_FFT_PACKED (see fft8192.cuh)
-#if DASP_FFT_PACKED
+// packed fp32x2 helpers of the generator's R-point DFT (FFMA2 / FMUL2, see fft8192.cuh)
 __device__ __forceinline__ float2 gen_ffma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 __device__ __forceinline__ float2 gen_fmul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
-#else
-__device__ __forceinline__ float2 gen_ffma2(float2 a, float2 b, float2 c) { return make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y)); }
-__device__ __forceinline__ float2 gen_fmul2(float2 a, float2 b) { return make_float2(a.x * b.x, a.y * b.y); }
-#endif
 
 // ---- spectral synthesis (device-noise mode) ------------------------------------------------------
 // The band-filtered noise only has to be a stationary Gaussian process with the FIR's autocovariance on
@@ -281,8 +278,8 @@ __device__ __forceinline__ float2 box_muller(unsigned a, unsigned b) {
 __constant__ float2 c_root[17][16];
 
 // One residue class pair (j1, nb - j1) of one band signal: draws the R bins of each class, runs the R-point
-// DFT + twiddle ladder and hands  Q_b[j1], Q_b[nb - j1]  (b = 0 .. R-1) to `emit(b, q_j1, q_mirror)`.
-// Shared by the stand-alone generator kernel and the fused synthesis kernel, so both produce the same stream.
+// DFT + twiddle ladder and hands  Q_b[j1], Q_b[nb - j1]  (b = 0 .. R-1) to `emit(b, q_j1, q_mirror)`, which
+// spectral_gen_kernel stores in the layout its consumer reads.
 template <int R, class Emit>
 __device__ __forceinline__ void spectral_unit(int j1, int nb, const float2* __restrict__ h, unsigned long long pair,
                                               const PhiloxKeys& keys, Emit&& emit) {
@@ -989,136 +986,6 @@ ifft_irgrad_kernel(const float* __restrict__ Epl, const float* __restrict__ twid
   }
 }
 
-// ---- fused IR synthesis (device-noise mode, nb == 8192, R <= 8) -------------------------------------
-// spectral_gen -> inverse FFT -> shape/accumulate as ONE kernel, so the 4.7 MB-per-item filtered-noise buffer is
-// written at most once (for the backward) instead of being written, transformed in place and read back.
-//
-// One thread-block CLUSTER of R CTAs per item; CTA c owns polyphase class c, i.e. the IR taps R a + c.
-//   * generation: the 12 * (nb/2 + 1) class pairs of the item are dealt round-robin over the R * 512 threads of
-//     the cluster (so every thread draws the same number of units); a unit's R results go to the R CTAs of the
-//     cluster as remote shared-memory stores (DSMEM) into the band's spectrum buffer G[band & 1] (planar re / im).
-//   * as soon as a band is complete (cluster barrier), every CTA runs the in-shared-memory inverse FFT of its
-//     class (fft8192.cuh) and accumulates  gain_k env_k(t) f_k(t) / 12  for its 16 taps per thread in registers;
-//     f is stored for the backward only when the caller keeps it.
-//   * G is double buffered by band parity: a second (split arrive / wait) cluster barrier hands a buffer back to
-//     the generators once every CTA has finished reading it (after FFT pass 2).
-constexpr int kMaxFusedR = 8;
-
-__device__ __forceinline__ unsigned cluster_ctarank() {
-  unsigned r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire;" ::: "memory"); }
-// generic pointer to the same shared-memory location in CTA `rank` of the cluster (DSMEM).  Kept 64-bit/generic on
-// purpose: with 32-bit shared::cluster addresses ptxas folded "+ 4 nb" of the mirror index into the store's
-// immediate AFTER widening (base - 4 j1) to 64 bits, which wraps for rank 0 and faults.
-__device__ __forceinline__ float* map_to_cta(float* smem_ptr, unsigned rank) {
-  uint64_t r;
-  asm volatile("mapa.u64 %0, %1, %2;" : "=l"(r) : "l"(reinterpret_cast<uint64_t>(smem_ptr)), "r"(rank));
-  return reinterpret_cast<float*>(r);
-}
-
-template <int R>
-__global__ void __launch_bounds__(kFusedThreads, 1)
-ir_synth_fused_kernel(const float2* __restrict__ H1, const float* __restrict__ twiddles,
-                      const float* __restrict__ params, float2* __restrict__ Hb, float2* __restrict__ Csave, int64_t item0, int64_t L, int64_t leff, int jb,
-                      const unsigned long long* seed) {
-  constexpr int nb = fft8k::kN, U = nb / 2 + 1, CT = R * kFusedThreads, total = kBands * U;
-  static_assert(CT < U, "at most one band may complete per generation round");
-  extern __shared__ __align__(16) float sm[];
-  float* G = sm;                                   // [parity][re, im][8192]
-  float* Yr = sm + 4 * fft8k::kPlaneG;
-  float* Yi = Yr + fft8k::kPlaneY;
-  float* tabf = Yi + fft8k::kPlaneY;
-  float* gk = tabf + fft8k::kTabFloats;
-  float* rk = gk + 16;
-  const int t = threadIdx.x;
-  const unsigned c = cluster_ctarank();
-  const int64_t il = blockIdx.y;
-
-  for (int e = t; e < fft8k::kTabFloats; e += kFusedThreads) tabf[e] = twiddles[e];
-  if (t < kBands) {
-    gk[t] = params[il * 25 + t] * (1.0f / kBands);
-    rk[t] = -(params[il * 25 + kBands + t] * 10.0f + 1.0f);
-  }
-  const fft8k::Tables tb = fft8k::carve_tables(tabf);
-  float* remote[R];                                // G of every CTA of the cluster
-#pragma unroll
-  for (int b = 0; b < R; ++b) remote[b] = map_to_cta(G, (unsigned)b);
-  const PhiloxKeys keys = philox_keys(__ldg(seed));
-  const float step = 1.0f / (float)(L - 1);
-  float accr[16], acci[16];
-#pragma unroll
-  for (int q = 0; q < 16; ++q) { accr[q] = 0.f; acci[q] = 0.f; }
-  // every CTA of the cluster must be resident (and its tables written) before the first remote store
-  cluster_arrive();
-  cluster_wait();
-
-  int processed = 0;
-  bool buffer_handed_back = false;                 // an arrive of the "G is free" barrier is outstanding
-  constexpr int rounds = (total + CT - 1) / CT;
-  for (int r = 0; r < rounds; ++r) {
-    if (buffer_handed_back) { cluster_wait(); buffer_handed_back = false; }
-    const int u = r * CT + (int)c * kFusedThreads + t;
-    if (u < total) {
-      const int k = u / U, j1 = u - k * U;
-      const unsigned long long pair = (unsigned long long)((item0 + il) * kBands + k);
-      const bool self_mirror = (j1 == 0) || (2 * j1 == nb);
-      const int off = (k & 1) * 2 * fft8k::kPlaneG;
-      spectral_unit<R>(j1, nb, H1 + (int64_t)k * (R * nb / 2 + 1), pair, keys, [&](int b, float2 q, float2 qm) {
-        float* base = remote[b] + off;
-        base[j1] = q.x;
-        base[fft8k::kPlaneG + j1] = q.y;
-        if (!self_mirror) {
-          base[nb - j1] = qm.x;
-          base[fft8k::kPlaneG + nb - j1] = qm.y;
-        }
-      });
-    }
-    const int done = (r + 1) * CT < total ? (r + 1) * CT : total;
-    if (done / U > processed) {                    // band `processed` is complete in every CTA's G
-      cluster_arrive();
-      cluster_wait();
-      const int kk = processed;
-      float* gr = G + (kk & 1) * 2 * fft8k::kPlaneG;
-      float* gi = gr + fft8k::kPlaneG;
-      fft8k::p1<true>(gr, gi, tb, t);
-      __syncthreads();
-      fft8k::p2<true>(gr, gi, Yr, Yi, tb, t);
-      __syncthreads();
-      cluster_arrive();                            // this CTA no longer reads G[kk & 1]
-      buffer_handed_back = true;
-      fft8k::P3Regs q3;
-      fft8k::p3_load<true>(Yr, Yi, t, q3);
-      __syncthreads();
-      fft8k::p3_store<true>(Yr, Yi, tb, t, q3);
-      __syncthreads();
-      float xr[16], xi[16];
-      fft8k::p4<true>(Yr, Yi, t, xr, xi);
-      const float g = gk[kk], rr = rk[kk];
-      float2* fout = Csave ? Csave + ((il * kBands + kk) * R + c) * (int64_t)nb : nullptr;
-#pragma unroll
-      for (int q = 0; q < 16; ++q) {
-        const int a = t + 512 * q;
-        const float e = g * __expf(rr * time_axis((int64_t)R * a + c, L, step));
-        accr[q] = fmaf(e, xr[q], accr[q]);
-        acci[q] = fmaf(e, xi[q], acci[q]);
-        if (fout) fout[a] = make_float2(xr[q], xi[q]);
-      }
-      ++processed;     // (Y is next written by pass 2 of the following band, behind a cluster barrier)
-    }
-  }
-  if (buffer_handed_back) cluster_wait();
-  float2* out = Hb + il * (int64_t)jb * kNbA;
-#pragma unroll
-  for (int q = 0; q < 16; ++q) {
-    const int64_t tau = (int64_t)R * (t + 512 * q) + c;
-    if (tau < leff) out[(tau / kB) * kNbA + (tau % kB)] = make_float2(accr[q], acci[q]);
-  }
-}
-
 // part[((item*nparts + blockIdx.x)*12 + k)*2 + {0,1}], nparts = gridDim.x; threads stride over time
 __global__ void ir_grad_pp_kernel(const float2* __restrict__ Et, const float2* __restrict__ C,
                                   const float* __restrict__ params, float* __restrict__ part, int64_t L, int64_t leff,
@@ -1579,8 +1446,6 @@ bool dispatch_spectral(int R, float2* C, const float2* H1, int64_t item0, int64_
 }
 constexpr int kMaxSpectralR = 16;
 
-// fused synthesis: one cluster of R CTAs per item.  Returns false when the device cannot co-schedule such a
-// cluster (then the three-kernel path is used), true after a launch attempt (check cudaGetLastError).
 // twiddle tables of fft8192.cuh (fp64 on the host, once per device)
 std::map<int, float*> g_fft_tab;
 int get_fft_tables(cudaStream_t st, const float** out) {
@@ -1617,48 +1482,7 @@ int launch_ifft_shape(float2* C, const float* tw, const float* params, float2* h
   DASP_LAUNCH_OK("ifft_shape_kernel");
   return DASP_OK;
 }
-int g_last_fused = 0;                                // test hook: IR-synthesis path of the last forward chunk
-std::map<std::pair<int, int>, int> g_fused_ok;      // (device, R) -> clusters that fit, guarded by g_mu
-template <int R>
-bool launch_fused(const float2* H1, const float* tw, const float* params, float2* hs, float2* Csave, int64_t item0, int64_t items,
-                  int64_t L, int64_t leff, int jb, const unsigned long long* seed, cudaStream_t st) {
-  auto kern = ir_synth_fused_kernel<R>;
-  const size_t smem = sizeof(float) * kFusedSmemFloats;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(R, (unsigned)items, 1);
-  cfg.blockDim = dim3(kFusedThreads, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = R; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  auto it = g_fused_ok.find({dev, R});
-  if (it == g_fused_ok.end()) {
-    int n = 0;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-        cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) {
-      n = 0;
-      cudaGetLastError();
-    }
-    it = g_fused_ok.emplace(std::make_pair(dev, R), n).first;
-  }
-  if (it->second < 1) return false;
-  cudaLaunchKernelEx(&cfg, kern, H1, tw, params, hs, Csave, item0, L, leff, jb, seed);
-  return true;
-}
-bool dispatch_fused(int R, const float2* H1, const float* tw, const float* params, float2* hs, float2* Csave, int64_t item0,
-                    int64_t items, int64_t L, int64_t leff, int jb, const unsigned long long* seed, cudaStream_t st) {
-  switch (R) {
-#define DASP_R(r) case r: return launch_fused<r>(H1, tw, params, hs, Csave, item0, items, L, leff, jb, seed, st);
-    DASP_R(1) DASP_R(2) DASP_R(3) DASP_R(4) DASP_R(5) DASP_R(6) DASP_R(7) DASP_R(8)
-#undef DASP_R
-    default: return false;
-  }
-}
+int g_last_path = 0;                                 // test hook: IR-synthesis path of the last forward chunk
 
 struct Plans { PlanVal blk_c2c, pp_c2c, xi_c2c, hj_c2c; size_t work; };
 int get_plans(const Geom& g, int64_t items, Plans& p) {
@@ -1749,7 +1573,7 @@ using namespace dasp;
 
 extern "C" {
 
-int dasp_debug_reverb_last_path(void) { return g_last_fused; }
+int dasp_debug_reverb_last_path(void) { return g_last_path; }
 
 // host-side restatement of signal.octave_band_filterbank: writes 12*taps floats (no GPU needed)
 int dasp_reverb_filterbank(int64_t taps, double sample_rate, float* out) {
@@ -1846,29 +1670,16 @@ int dasp_reverb_fwd(const float* x, int64_t in_chs, const float* params, const f
 
     // ---- IR synthesis: (left, right) taps land in the zero-initialised partition layout hs ----
     DASP_CUDA_OK(cudaMemsetAsync(hs, 0, sizeof(float2) * items * J * kNbA, st));
-    // device-noise IR synthesis, three variants (same Philox stream, so they agree to transform rounding):
-    //   2 = generator -> ifft_shape_kernel (own in-shared-memory FFT fused with the shaping; default for nb == 8192)
-    //   1 = one thread-block cluster per item (generator + FFT + shaping in one kernel; dasp_debug_reverb_path(2))
-    //   0 = generator -> batched cuFFT -> shape_ir_pp_kernel (dasp_debug_reverb_path(1), and any other nb)
-    int synth = 0;
+    // device-noise IR synthesis (the same Philox stream on both paths):
+    //   nb == 8192: generator -> ifft_shape_kernel (own in-shared-memory FFT fused with the shaping)
+    //   other nb  : generator -> batched cuFFT -> shape_ir_pp_kernel
     const bool own_fft = spectral && nb == fft8k::kN && g.L < (int64_t)1 << 31;
-    if (own_fft && debug_reverb_path() == 2 && g.rpp <= kMaxFusedR) synth = 1;
-    else if (own_fft && debug_reverb_path() != 1) synth = 2;
     // audio convolution: block transforms on the own FFT (fused with their pre/post kernels) when the rows allow bulk copies
-    const bool own_conv = debug_reverb_path() != 1 && (n % 4 == 0) && aligned16(x);
+    const bool own_conv = (n % 4 == 0) && aligned16(x);
     const float* tw = nullptr;
-    if ((synth != 0 || own_conv) && (rc = get_fft_tables(st, &tw)) != DASP_OK) return rc;
-    if (synth == 1) {
-      if (dispatch_fused((int)g.rpp, H1, tw, params + item0 * 25, hs, f_save ? C : nullptr, item0, items, g.L, g.leff, J,
-                         seed, st)) {
-        DASP_LAUNCH_OK("ir_synth_fused_kernel");
-      } else {
-        synth = 2;                                   // the device cannot co-schedule such a cluster
-      }
-    }
-    g_last_fused = synth;
-    if (synth == 1) {
-    } else if (synth == 2) {
+    if ((own_fft || own_conv) && (rc = get_fft_tables(st, &tw)) != DASP_OK) return rc;
+    g_last_path = own_fft ? 2 : 0;
+    if (own_fft) {
       dispatch_spectral((int)g.rpp, C, H1, item0, items, nb, seed, /*planar=*/true, st);
       DASP_LAUNCH_OK("spectral_gen_kernel");
       if ((rc = launch_ifft_shape(C, tw, params + item0 * 25, hs, f_save != nullptr, items, g, J, st)) != DASP_OK) return rc;
@@ -1970,9 +1781,8 @@ int dasp_reverb_bwd(const float* gy, const float* x, int64_t in_chs, const float
     const float2* xs = (const float2*)xspec_save + item0 * I * (int64_t)kNbA;
     const float2* hs = (const float2*)irspec_save + item0 * J * (int64_t)kNbA;
 
-    // block transforms on the own in-shared-memory FFT (fused with their neighbours) when the rows allow bulk copies;
-    // dasp_debug_reverb_path(1) pins the cuFFT pipeline (the two are compared by the tests)
-    const bool own_conv = debug_reverb_path() != 1 && (n % 4 == 0) && aligned16(gy);
+    // block transforms on the own in-shared-memory FFT (fused with their neighbours) when the rows allow bulk copies
+    const bool own_conv = (n % 4 == 0) && aligned16(gy);
     const bool own_irgrad = own_conv && polyphase && nb == fft8k::kN && g.L < (int64_t)1 << 31;
     const float* tw = nullptr;
     if (own_conv) {

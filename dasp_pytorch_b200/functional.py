@@ -530,13 +530,11 @@ def parametric_eq_packed(x: torch.Tensor, sample_rate: float, params: torch.Tens
 # noise-shaped reverberation
 # --------------------------------------------------------------------------------------
 
-import os as _os
-
 # Items per pass of the reverb pipeline (bounds the workspace).  Default: one item per SM of the device, so that the
 # one-CTA-per-SM FFT kernels run in whole waves (ifft_shape_kernel: R CTAs per item -> exactly R waves; the persistent
 # block-transform kernels: the same number of blocks per CTA).  Measured on B200 (148 SMs), chain step at batch 1024:
-# 74 -> 14.83 ms, 128 -> 14.61 ms, 148 -> 14.11 ms.  Override for experiments with DASP_REVERB_CHUNK.
-REVERB_CHUNK_ITEMS = int(_os.environ.get("DASP_REVERB_CHUNK", "0"))      # 0 = automatic
+# 74 -> 14.83 ms, 128 -> 14.61 ms, 148 -> 14.11 ms.  A positive value overrides the default.
+REVERB_CHUNK_ITEMS = 0      # 0 = automatic
 
 
 def reverb_chunk_items(device) -> int:

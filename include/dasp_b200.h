@@ -45,17 +45,12 @@ int dasp_compiled_arch(void);
 void dasp_shutdown(void);
 /* The dasp_debug_* entry points are TEST HOOKS: process-global switches, not thread-safe, not for production
  * callers (they exist so that every kernel variant can be pinned against the oracle at small sizes). */
-/* test hook: pin the warps-per-row variant of the scan kernels (1, 2, 3, 4, 8, 16; 0 = automatic choice; a kernel
- * family without the requested variant keeps its automatic choice) */
+/* test hook: pin the warps-per-row variant of the scan kernels (1, 2, 4, 8, 16; 0 = automatic choice).  The EQ
+ * forward has 4, 8 and 16, the EQ backward a single variant, the compressor all five; a kernel family without the
+ * requested variant keeps its automatic choice */
 void dasp_debug_force_warps(int warps);
-/* test hook: pin the number of x / dL/dy stages per warp of the EQ backward (1 or 2; 0 = automatic) */
-void dasp_debug_eq_bwd_stages(int stages);
-/* test hook, IR synthesis of the device-noise reverb (all variants draw the same Philox stream and must agree):
-   0 = automatic (generator -> fused in-shared-memory inverse FFT + shaping kernel when the block FFT is 8192 points),
-   1 = generator -> batched cuFFT -> shaping kernel, 2 = one thread-block-cluster kernel per item */
-void dasp_debug_reverb_path(int path);
-/* test hook: variant used by the last chunk of the most recent dasp_reverb_fwd: 0 = cuFFT pipeline, 1 = cluster
-   kernel, 2 = generator + fused FFT/shaping kernel */
+/* test hook: IR synthesis used by the last chunk of the most recent dasp_reverb_fwd: 0 = cuFFT pipeline (or the
+   caller's noise tensor), 2 = generator + own in-shared-memory FFT/shaping kernel (device noise, 8192-point blocks) */
 int dasp_debug_reverb_last_path(void);
 
 /* test hook: 1 = the spectral IR synthesis uses unit-impulse filters, so the f_save buffer of dasp_reverb_fwd

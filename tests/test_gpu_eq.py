@@ -72,21 +72,19 @@ def test_eq_ragged_shapes(cuda_device, bs, chs, n):
     _check(cuda_device, x, denorm(p01, eq_ranges()), tail=1 << 16)
 
 
-@pytest.mark.parametrize("warps,stages", [(1, 1), (1, 2), (2, 1), (2, 2), (3, 1), (3, 2), (4, 1), (4, 2), (8, 1), (16, 1), (16, 2)])
-def test_eq_every_warps_per_pair_variant(cuda_device, warps, stages):
-    """the kernels pick 1/2/4/8 warps per row pair from the batch size (warp w owns tiles w, w+W, ...; carries travel
-    through mbarrier-guarded mailboxes) and 1 or 2 load stages in the backward; pin each variant (test hooks) on a
-    small batch with many tiles per warp, a ragged tail and an odd number of rows, so that every instantiation runs
-    at a size the oracle checks in seconds"""
+@pytest.mark.parametrize("warps,chs", [(4, 1), (4, 2), (8, 1), (8, 2), (16, 1), (16, 2)])
+def test_eq_every_warps_per_pair_variant(cuda_device, warps, chs):
+    """the forward picks 4/8/16 warps per row pair from the batch size (warp w owns tiles w, w+W, ...; carries travel
+    through mbarrier-guarded mailboxes); pin each variant (test hook) with both coefficient-table types (odd channel
+    counts pair rows of different items) on a small batch with many tiles per warp, a ragged tail and an odd number of
+    rows, so that every instantiation runs at a size the oracle checks in seconds"""
     from dasp_pytorch_b200 import _abi
-    x, p01 = _inputs(3, 1 if warps in (3, 4) and stages == 1 else 2, 480 * 8 * 3 + 100, seed=14, low_corner=(warps == 2))
+    x, p01 = _inputs(3, chs, 480 * 8 * 3 + 100, seed=14, low_corner=(warps == 8))
     _abi.lib().dasp_debug_force_warps(warps)
-    _abi.lib().dasp_debug_eq_bwd_stages(stages)
     try:
         _check(cuda_device, x, denorm(p01, eq_ranges()), tail=1 << 16, strict=True)
     finally:
         _abi.lib().dasp_debug_force_warps(0)
-        _abi.lib().dasp_debug_eq_bwd_stages(0)
 
 
 def test_eq_is_deterministic_and_warp_count_invariant(cuda_device):
@@ -98,7 +96,7 @@ def test_eq_is_deterministic_and_warp_count_invariant(cuda_device):
     xs = x.to(cuda_device)
     ps = [p.to(cuda_device) for p in denorm(p01, eq_ranges())]
     outs = []
-    for w in (1, 2, 3, 4, 8, 16, 2):          # 16 exists for the forward only (the backward keeps its own choice)
+    for w in (4, 8, 16, 4):                   # the backward has a single variant
         _abi.lib().dasp_debug_force_warps(w)
         try:
             xx = xs.clone().requires_grad_(True)

@@ -174,53 +174,6 @@ def test_reverb_contract(cuda_device):
     assert torch.equal(y1, y2)
 
 
-@pytest.mark.parametrize("n,L", [(4000, 6000), (12000, 30000), (20000, 20000), (30000, 40000), (36000, 36000),
-                                 (48000, 96000), (50000, 50000), (60000, 60000), (70000, 80000)])
-def test_reverb_ir_synthesis_variants_agree(cuda_device, n, L):
-    """Three device implementations of the device-noise IR synthesis draw the same Philox stream, so for one seed they
-    must agree to transform rounding -- output, saved filtered noise (through the parameter gradients) and dL/dx:
-      0: generator -> batched cuFFT -> shaping kernel,
-      2: generator -> own in-shared-memory 8192-point inverse FFT fused with the shaping (the default),
-      1: one thread-block cluster of R CTAs per item doing all three steps (R <= 8).
-    The cases cover polyphase factors R = 1 ... 9."""
-    import dasp_pytorch_b200 as D
-    from dasp_pytorch_b200 import _abi
-    bs, taps = 3, 1023
-    R = -(-(min(n, L) + taps - 1) // 8192)
-    g = torch.Generator().manual_seed(n)
-    x = (torch.rand(bs, 2, n, generator=g) * 2 - 1).to(cuda_device)
-    x[0, :, 1:] = 0.0                                          # item 0: an impulse -> its wet signal is the IR itself
-    w = torch.randn(bs, 2, n, generator=g).to(cuda_device)
-    p = [q.to(cuda_device) for q in _params01(bs, 3)]
-    p[24] = torch.full((bs,), 0.9, device=cuda_device)
-
-    def run(path):
-        _abi.lib().dasp_debug_reverb_path(path)
-        try:
-            torch.manual_seed(77)
-            xx = x.clone().requires_grad_(True)
-            pp = [q.clone().requires_grad_(True) for q in p]
-            y = D.noise_shaped_reverberation(xx, SR, *pp, num_samples=L, num_bandpass_taps=taps)
-            used = _abi.lib().dasp_debug_reverb_last_path()
-            (y * w).sum().backward()
-            torch.manual_seed(77)
-            with torch.no_grad():                               # forward that keeps nothing for a backward
-                y_inf = D.noise_shaped_reverberation(x, SR, *p, num_samples=L, num_bandpass_taps=taps)
-            assert torch.equal(y.detach(), y_inf)
-            return used, y.detach(), xx.grad, torch.stack([q.grad for q in pp], 1)
-        finally:
-            _abi.lib().dasp_debug_reverb_path(0)
-
-    used_ref, y_ref, dx_ref, dp_ref = run(1)
-    assert used_ref == 0 and y_ref.abs().max() > 1e-3
-    for path, expect in ((0, 2), (2, 1 if R <= 8 else 2)):
-        used, y, dx, dp = run(path)
-        assert used == expect, (path, used)
-        assert peak_err(y, y_ref).max() < 2e-5, (path, peak_err(y, y_ref))
-        assert peak_err(dx, dx_ref).max() < 2e-5, (path, peak_err(dx, dx_ref))
-        assert float((dp - dp_ref).abs().max() / dp_ref.abs().max()) < 2e-5, path
-
-
 def test_reverb_chunking_is_invisible(cuda_device, monkeypatch):
     """The pipeline processes the batch in chunks (default: one item per SM); the Philox stream is keyed by the
     absolute item index, so any chunk size -- including one that leaves a remainder chunk -- gives the same result."""
@@ -247,27 +200,34 @@ def test_reverb_chunking_is_invisible(cuda_device, monkeypatch):
             assert float((a - b).abs().max() / b.abs().max()) < 2e-6, chunk
 
 
-@pytest.mark.parametrize("n,L,taps,want_r", [(6000, 4000, 255, 1), (48000, 48000, 1023, 6), (48000, 96000, 1023, 6),
-                                             (70000, 66000, 1023, 9)])
+@pytest.mark.parametrize("n,L,taps,want_r", [(6000, 4000, 255, 1), (12000, 30000, 1023, 2), (20000, 20000, 1023, 3),
+                                             (30000, 40000, 1023, 4), (36000, 36000, 1023, 5), (48000, 48000, 1023, 6),
+                                             (48000, 96000, 1023, 6), (50000, 50000, 1023, 7), (60000, 60000, 1023, 8),
+                                             (70000, 66000, 1023, 9), (20000, 20000, 2047, 2), (6001, 9000, 255, 1)])
 def test_reverb_device_noise_path_pinned_to_oracle(cuda_device, n, L, taps, want_r):
-    """DETERMINISTIC parity of the DEFAULT (benchmarked) device-noise path -- spectral_gen_kernel -> ifft_shape_kernel
-    -> partitioned convolution, and its backward incl. ir_grad_pp_kernel -- against the fp64 oracle.
+    """DETERMINISTIC parity of the device-noise path against the fp64 oracle, for polyphase factors R = 1 ... 9:
+    spectral_gen_kernel -> ifft_shape_kernel (8192-point blocks) or -> batched cuFFT -> shape_ir_pp_kernel (2047 taps:
+    16384-point blocks), then the partitioned convolution (own FFT, or cuFFT for the unaligned n = 6001), and the
+    backward incl. ir_grad_pp_kernel.
 
-    The generator draws, per (item, band, channel), a white PERIODIC sequence w of length n1 = R*8192 in the frequency
+    The generator draws, per (item, band, channel), a white PERIODIC sequence w of length n1 = R*nb in the frequency
     domain and filters it circularly: f[t] = sum_m h[m] w[(t-m) mod n1].  With the test hook
     dasp_debug_reverb_flat_filterbank the filters are unit impulses, so the f buffer kept for the backward is w itself.
     The reference-style noise tensor  noise[t'] = w[(t' - P) mod n1]  (P = taps-1, h symmetric) then makes the
     reference's valid cross-correlation (functional.py:551-556) produce exactly the same f for every t < min(L, n)
     (n1 >= min(L, n) + P: no wrap-around inside the window), so y, dL/dx and all 25 parameter gradients of the default
     call must equal oracle.noise_shaped_reverberation(noise=...) to 1e-4 -- a wrong Hermitian pairing, twiddle,
-    s_half/s_full scaling or polyphase index anywhere in the benchmarked kernels fails this test."""
+    s_half/s_full scaling or polyphase index anywhere in these kernels fails this test."""
     import dasp_pytorch_b200 as D
     from dasp_pytorch_b200 import _abi
     lib = _abi.lib()
-    bs, P, nb = 2, taps - 1, 8192
-    leff = min(L, n)
-    R = -(-(leff + P) // nb)
+    bs, P = 2, taps - 1
+    geom = _abi.ReverbGeom()
+    assert lib.dasp_reverb_geometry(0, n, L, taps, 0, geom) == 0
+    nb, R = geom.nb, geom.rpp
     assert R == want_r
+    want_path = 0 if taps == 2047 else 2        # 2047 taps need 16384-point blocks: the cuFFT polyphase synthesis
+    assert nb == (16384 if want_path == 0 else 8192)
     n1 = R * nb
     g = torch.Generator().manual_seed(n + L)
     x = (torch.rand(bs, 2, n, generator=g) * 2 - 1)
@@ -283,7 +243,7 @@ def test_reverb_device_noise_path_pinned_to_oracle(cuda_device, n, L, taps, want
         fsave = yq.grad_fn.saved_tensors[3]
     finally:
         lib.dasp_debug_reverb_flat_filterbank(0)
-    assert lib.dasp_debug_reverb_last_path() == 2                      # generator + fused FFT/shaping kernel
+    assert lib.dasp_debug_reverb_last_path() == want_path
     w = torch.view_as_complex(fsave[: bs * 12 * R * nb * 2].reshape(bs, 12, R, nb, 2).contiguous())   # [.., b, a] = w[R a + b]
     w = w.permute(0, 1, 3, 2).reshape(bs, 12, n1).cpu()               # (item, band, t), real = left, imag = right
     assert abs(float(w.real.std()) - 1.0) < 0.02 and abs(float(w.imag.std()) - 1.0) < 0.02      # white, unit variance
@@ -296,10 +256,15 @@ def test_reverb_device_noise_path_pinned_to_oracle(cuda_device, n, L, taps, want
         return D.noise_shaped_reverberation(xx, SR, *p, **kw)
 
     y, dx, dp = run_with_grads(run_default, x, params, torch.float32, cuda_device)
-    assert lib.dasp_debug_reverb_last_path() == 2
+    assert lib.dasp_debug_reverb_last_path() == want_path
     y64, dx64, dp64 = run_with_grads(
         lambda xx, p: oracle.noise_shaped_reverberation(xx, SR, *p, noise=noise, method="fft", **kw),
         x, params, torch.float64, "cpu")
     assert peak_err(y, y64).max() < TOL, peak_err(y, y64)
     assert peak_err(dx, dx64).max() < TOL, peak_err(dx, dx64)
     assert param_grad_err(dp, dp64).max() < TOL, param_grad_err(dp, dp64)
+
+    # 3) a forward that keeps nothing for a backward computes the same bits
+    with torch.no_grad():
+        y_inf = run_default(x.to(cuda_device), [p.to(cuda_device) for p in params])
+    assert torch.equal(y_inf.cpu(), y)
